@@ -64,7 +64,31 @@ def parse():
     ap.add_argument("--nvtx", action="store_true", help="wrap the LAST step of the steady-state run in an NVTX range "
                     "'mdb_step' (ncu --nvtx --nvtx-include 'mdb_step/' then profiles exactly one step)")
     ap.add_argument("--tune", default="", help="experiments: launch heuristics as k=v[,k=v] (keys of ops.tuning)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write x_prev and pred_x0 of the last timed step (rank 0's frames of "
+                         "the headline run) as DIR/<name>.npy in float32, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(path, arrays):
+    """name -> tensor, written as path/<name>.npy (float32).  Past DUMP_BYTES in all (headers included), each array is
+    replaced by the same fixed, seeded sample of its flattened elements, so that dumps of one configuration compare."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    budget = DUMP_BYTES - 256 * len(arrays)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > budget:
+            keep = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -133,7 +157,8 @@ def host_threads():
 
 
 def cpu_port_step_seconds(sd, latent, steps, warmup, torch):
-    """Times the oracle port of p_sample_ddim (oracle/restatement.py) on the host cores."""
+    """Times the oracle port of p_sample_ddim (oracle/restatement.py) on the host cores: the mean step time and the
+    x_prev / pred_x0 of the last step."""
     from oracle import restatement as R  # the ONE place bench.py executes oracle/: the CPU baseline
     from magicdance_b200 import synth
     import numpy as np
@@ -147,12 +172,13 @@ def cpu_port_step_seconds(sd, latent, steps, warmup, torch):
             t = torch.full((1,), int(sched["timesteps"][index]), dtype=torch.long)
             t0 = time.perf_counter()
             # as executed by the reference: appearance + pose + UNet-read, then pose (discarded) + UNet-uc
-            x_prev, _, _, _ = R.p_sample_ddim(sd, x, t, index, inp["context"], inp["pose"], inp["ref"], sched, scale=7.0)
+            x_prev, pred_x0, _, _ = R.p_sample_ddim(sd, x, t, index, inp["context"], inp["pose"], inp["ref"], sched,
+                                                    scale=7.0)
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
             x = x_prev
-    return sum(times) / len(times)
+    return sum(times) / len(times), {"x_prev": x_prev, "pred_x0": pred_x0}
 
 
 def run_reference(args):
@@ -164,9 +190,11 @@ def run_reference(args):
     torch.set_grad_enabled(False)
     torch.set_num_threads(host_threads())
     sd = synth.synth_state_dict(seed=0)
-    steps = max(1, min(args.steps, int(os.environ.get("MDB_REF_MAX_STEPS", "2"))))
+    steps = args.steps
     warm = 1 if args.warmup > 0 else 0
-    sec = cpu_port_step_seconds(sd, args.latent, steps, warm, torch)
+    sec, outputs = cpu_port_step_seconds(sd, args.latent, steps, warm, torch)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     val = 1.0 / sec
     sample = (f"{steps} timed p_sample_ddim step(s) of the 50-step chain (+{warm} warm-up), B=1, fp32, latent "
               f"{args.latent}x{args.latent}; per-step time extrapolates linearly to the chain")
@@ -351,6 +379,8 @@ class Bench:
         e1.record()
         self.barrier()
         launches = ops.launch_count() + gd.replayed_launches - l0
+        # what the last timed step hands its caller (the runs below overwrite these buffers)
+        self.outputs = {"x_prev": gd.x_prev.clone(), "pred_x0": gd.pred_x0.clone()}
         sec = self.max_over_ranks(e0.elapsed_time(e1)) * 1e-3
         clk = clocks.stop()
         bank_ms = self.max_over_ranks(timing["build0"].elapsed_time(timing["build1"]))
@@ -506,6 +536,7 @@ def run_ours(args):
     K, W, B = args.steps, args.warmup, args.batch
     # N > 1: the ranks hold frames of ONE sequence (shared reference image / prompt / x_T, own pose maps)
     main = b.measure(B, K, W, e2e=not args.no_e2e, sequence_frames=world > 1)
+    outputs = b.outputs
     roof = None
     if rank == 0 and not args.no_roofline:
         roof = b.roofline(B)
@@ -529,6 +560,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
     line = {
         "metric": METRIC, "value": main["value"], "unit": UNIT, "n_gpus": world, "steps": K, "warmup": max(W, 1),
@@ -570,7 +603,7 @@ def run_ours(args):
         torch.set_num_threads(host_threads())
         sd = {k: v.detach().float().cpu() for k, v in b.model.state_dict().items()
               if k.startswith(("model.diffusion_model.", "appearance_control_model.", "pose_control_model."))}
-        csec = cpu_port_step_seconds(sd, args.latent, 1, 0, torch)
+        csec, _ = cpu_port_step_seconds(sd, args.latent, 1, 0, torch)
         line["cpu_baseline"] = {"value": 1.0 / csec, "unit": UNIT, "cores": torch.get_num_threads(), "kind": "port",
                                 "sample": "1 p_sample_ddim step (index 49) of the same chain, B=1, fp32, as executed "
                                           "by the reference (incl. its discarded 2nd pose pass), no warm-up"}
