@@ -1,6 +1,6 @@
 """Per-kernel numerics cases: each function runs one C-ABI kernel on the GPU and returns
-(error, tolerance, description) against a plain PyTorch fp32 reference of the same op computed
-from the SAME fp16-rounded inputs.  Shared by tests/test_kernels_gpu.py and scripts/gpu_diag.py."""
+(error, tolerance, description) against a plain PyTorch fp32 or float64 reference of the same op
+computed from the SAME fp16-rounded inputs.  Shared by tests/test_kernels_gpu.py and scripts/gpu_diag.py."""
 import math
 
 import torch
@@ -219,66 +219,208 @@ def case_layernorm(rows, c, seed=0):
     return rel(out.float(), ref), 1.5e-3, f"layernorm rows={rows} c={c}"
 
 
-def case_attention(batch, heads, d, nq, n0, n1=0, kv1_batches=1, bank_batches=None, ldv_pad=False, seed=0):
-    c = heads * d
-    q = _rand(batch * nq, c, seed=seed).half()
-    k0 = _rand(batch * n0, c, seed=seed + 1).half()
-    v0 = _rand(batch * n0, c, seed=seed + 2).half()
-    ldv = (n0 + 7) // 8 * 8 if ldv_pad else n0
-    vt0 = torch.zeros(c, batch * ldv, dtype=torch.float16, device=DEV)
+ATT_BKV = 64       # keys per tile of every attention kernel (csrc/attention.cu, BKV)
+ATT_LAZY_LOG2 = 8  # the running max moves only when a tile's max exceeds it by more than this (log2 units)
+V_PAD_FILL = 3e4   # V^T columns [n, ldv) of a padded layout: large and finite, so a masked key with P != 0 shows
+
+
+def _vt_padded(v, batches, n, ldv):
+    """V [batches*n, c] -> V^T [c, batches*ldv]; padding columns hold +-V_PAD_FILL (the kernel must give them P = 0)"""
+    c = v.shape[1]
+    vt = torch.full((c, batches, ldv), V_PAD_FILL, dtype=torch.float16, device=v.device)
+    vt[1::2] = -V_PAD_FILL
+    vt[:, :, :n] = v.reshape(batches, n, c).permute(2, 0, 1)
+    return vt.reshape(c, batches * ldv)
+
+
+def attention_keys(b, k0, v0, n0, kv0_batches, k1=None, v1=None, n1=0, kv1_batches=1, bank_batches=0):
+    """keys / values that batch element b attends to, in the kernels' tile order (source 0, then source 1)"""
+    s0 = slice(b * n0, (b + 1) * n0) if kv0_batches > 1 else slice(0, n0)
+    kk, vv = [k0[s0]], [v0[s0]]
+    if n1 and b < bank_batches:
+        s1 = slice(b * n1, (b + 1) * n1) if kv1_batches > 1 else slice(0, n1)
+        kk.append(k1[s1])
+        vv.append(v1[s1])
+    return torch.cat(kk, 0), torch.cat(vv, 0)
+
+
+def attention_ref(q, heads, d, batch, nq, **kv):
+    """float64 softmax(q k^T / sqrt(d)) v per batch element from the same fp16 operands; kv: attention_keys' keywords"""
+    refs = []
     for b in range(batch):
-        vt0[:, b * ldv:b * ldv + n0] = v0[b * n0:(b + 1) * n0].t()
-    kw = {}
+        kk, vv = attention_keys(b, **kv)
+        qq = q[b * nq:(b + 1) * nq].double().reshape(nq, heads, d).transpose(0, 1)
+        kk = kk.double().reshape(-1, heads, d).transpose(0, 1)
+        vv = vv.double().reshape(-1, heads, d).transpose(0, 1)
+        s = (qq @ kk.transpose(1, 2)) * d ** -0.5
+        refs.append((s.softmax(-1) @ vv).transpose(0, 1).reshape(nq, heads * d))
+    return torch.cat(refs, 0)
+
+
+def case_attention(batch, heads, d, nq, n0, n1=0, kv1_batches=1, bank_batches=None, ldv_pad=False, mode="", seed=0):
+    """mode: '+'-joined layout options of the hot path —
+    qk_fused   Q and K0 are the two column halves of one [B*N, 2c] projection (self-attention, engine.py attn1);
+    shared_kv  one key/value set for the whole batch (kv0_batches = 1: the text context, engine.py attn2);
+    wide_out   the output is a column slice of a wider buffer (ldo > heads*d); its other columns stay untouched."""
+    modes = set(filter(None, mode.split("+")))
+    assert modes <= {"qk_fused", "shared_kv", "wide_out"}, modes
+    c = heads * d
+    kvb = 1 if "shared_kv" in modes else batch
+    if "qk_fused" in modes:
+        assert n0 == nq and kvb == batch
+        qk = _rand(batch * nq, 2 * c, seed=seed).half()
+        q, k0 = qk[:, :c], qk[:, c:]
+    else:
+        q = _rand(batch * nq, c, seed=seed).half()
+        k0 = _rand(kvb * n0, c, seed=seed + 1).half()
+    v0 = _rand(kvb * n0, c, seed=seed + 2).half()
+    ldv = (n0 + 7) // 8 * 8 if ldv_pad else n0
+    vt0 = _vt_padded(v0, kvb, n0, ldv)
+    kw, kv = {}, dict(k0=k0, v0=v0, n0=n0, kv0_batches=kvb)
+    bb = batch if bank_batches is None else bank_batches
     if n1:
         k1 = _rand(kv1_batches * n1, c, seed=seed + 3).half()
         v1 = _rand(kv1_batches * n1, c, seed=seed + 4).half()
-        kw = dict(k1=k1, vt1=v1.t().contiguous(), n1=n1, kv1_batches=kv1_batches,
-                  bank_batches=batch if bank_batches is None else bank_batches)
-    out = ops.attention(q, k0, vt0, n0, heads=heads, d=d, batch=batch, nq=nq, ldv0_batch=ldv, **kw)
-    refs = []
+        kw = dict(k1=k1, vt1=v1.t().contiguous(), n1=n1, kv1_batches=kv1_batches, bank_batches=bb)
+        kv.update(k1=k1, v1=v1, n1=n1, kv1_batches=kv1_batches, bank_batches=bb)
+    out, gap = None, 16
+    if "wide_out" in modes:
+        buf = torch.full((batch * nq, c + 3 * gap), 7.0, dtype=torch.float16, device=DEV)
+        out = buf[:, gap:gap + c]
+    res = ops.attention(q, k0, vt0, n0, heads=heads, d=d, batch=batch, nq=nq, out=out, kv0_batches=kvb,
+                        ldv0_batch=ldv, **kw)
+    err = rel(res.float(), attention_ref(q, heads, d, batch, nq, **kv))
+    if out is not None and not (torch.all(buf[:, :gap] == 7.0) and torch.all(buf[:, gap + c:] == 7.0)):
+        err = float("inf")  # wrote outside its column slice
+    return err, 3e-3, (f"attention B={batch} h={heads} d={d} nq={nq} n0={n0} n1={n1} "
+                       f"kv1b={kv1_batches} bank_b={bb} ldv={ldv} {mode}")
+
+
+# ---- attention logits that drive the online-softmax rescale path ---------------------------------------------------
+# With randn Q and K the logits are ~N(0, 1): after tile 0 no tile's max ever beats the running max by
+# ATT_LAZY_LOG2, so the O / l rescale and the re-emission of P (attn2/attn3's second pass) never run.  Here every
+# logit is placed: per head a unit direction u, q_i = a_i s u + r_i, k_j = t_j s u + r_j with the noise r
+# orthogonal to u and s^2 = sqrt(d) / log2(e), so the logit of row i and key j is a_i t_j + r_i.r_j / sqrt(d) in
+# log2 units (the noise is ~0.36 log2 units).  a_i (0 or 1) picks the peaky rows, t_j (log2 units) is the key profile.
+# tests/test_kernel_cases_cpu.py replays the kernels' per-row bookkeeping on these inputs and checks that each
+# pattern reaches the branch it claims.
+PEAKY_PATTERNS = ("rise", "slow_rise", "mixed_rows", "fall", "bank_peak", "ragged_peak")
+
+
+def _tile_ramp(j):
+    """-2 .. 0 across each 64-key tile: the softmax weight of a tile is spread over its keys, its max at the end"""
+    return -2.0 * (1.0 - (j % ATT_BKV).double() / (ATT_BKV - 1))
+
+
+def peaky_profiles(pattern, batch, nq, n0, n1):
+    """row amplitudes a [batch, nq] and key profiles t0 [batch, n0] (source 0), t1 [n1] (source 1, one bank)"""
+    a = torch.ones(batch, nq, dtype=torch.float64)
+    j0 = torch.arange(n0)
+    tile0 = (j0 // ATT_BKV).double()
+    t1 = torch.zeros(n1, dtype=torch.float64)
+    if pattern in ("rise", "mixed_rows"):
+        # steps of 12 and 18 alternately: a rescale on every tile; the optimistic P of an 18-step (2^18) overflows fp16
+        steps = torch.tensor([12.0 if i % 2 == 0 else 18.0 for i in range(int(tile0.max()) + 1)])
+        level = torch.cat([torch.zeros(1), steps.cumsum(0)[:-1]]).double()[j0 // ATT_BKV]
+        t0 = level + _tile_ramp(j0)
+        if pattern == "mixed_rows":
+            # in every 128-row Q tile: warp 1 rises, warp 2 stays flat, warps 0 and 3 rise on odd rows only —
+            # lanes of one warp and warps of one CTA disagree on the rescale vote
+            r = torch.arange(nq) % 128
+            w = r // 32
+            a[:] = torch.where(w == 1, 1.0, torch.where(w == 2, 0.0, (r % 2).double()))
+    elif pattern == "slow_rise":
+        # +5.5 per tile: every other tile is accepted against the old max (P up to ~2^6), the next one rescales
+        t0 = 5.5 * tile0 + _tile_ramp(j0)
+    elif pattern == "fall":
+        # max in tile 0; later tiles 30 .. ~150 log2 units below it (-32: room for the noise): P underflows to 0
+        # (ex2.approx.ftz, ex2_poly's clamp at -125)
+        t0 = torch.where(tile0 == 0, 0.0, -32.0 - 15.0 * (tile0 - 1)) + _tile_ramp(j0)
+    elif pattern == "bank_peak":
+        # source 0 flat, the peak in the bank: the rescale happens at the source boundary
+        t0 = _tile_ramp(j0)
+        j1 = torch.arange(n1)
+        t1 = 12.0 * (j1 // ATT_BKV + 1).double() + _tile_ramp(j1)
+    elif pattern == "ragged_peak":
+        # the peak in the last, partly valid tile (masked exponentials)
+        assert n0 % ATT_BKV
+        t0 = torch.where(tile0 == tile0.max(), 12.0, 0.0) + _tile_ramp(j0)
+    else:
+        raise ValueError(pattern)
+    t0 = t0.expand(batch, n0).clone()
+    if pattern == "ragged_peak":
+        # the last K tile of batch b runs on into the first keys of batch b+1: give those the largest logits of the
+        # whole tensor, so that a key past n0 that is not masked dominates batch b's output
+        t0[1:, :ATT_BKV - n0 % ATT_BKV] = 40.0
+    return a, t0, t1
+
+
+def attention_peaky_inputs(batch, heads, d, nq, n0, n1, pattern, bank_batches, seed=0, device=None):
+    """fp16 operands of one peaky attention case (K/V per batch element for source 0, one shared bank for source 1)"""
+    device = DEV if device is None else device
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    c = heads * d
+    a, t0, t1 = peaky_profiles(pattern, batch, nq, n0, n1)
+    u = torch.randn(heads, d, generator=g, dtype=torch.float64)
+    u = u / u.norm(dim=1, keepdim=True)
+    s = (d ** 0.5 / math.log2(math.e)) ** 0.5
+
+    def build(amp):  # amp [rows] -> [rows, heads*d]: amp s u + noise orthogonal to u, per head
+        r = 0.5 * torch.randn(amp.shape[0], heads, d, generator=g, dtype=torch.float64)
+        r = r - (r * u).sum(-1, keepdim=True) * u
+        return (amp[:, None, None] * s * u + r).reshape(-1, c).half().to(device)
+
+    q = build(a.reshape(-1))
+    k0 = build(t0.reshape(-1))
+    v0 = torch.randn(batch * n0, c, generator=g).half().to(device)
+    k1 = build(t1) if n1 else None
+    v1 = torch.randn(n1, c, generator=g).half().to(device) if n1 else None
+    kv = dict(k0=k0, v0=v0, n0=n0, kv0_batches=batch, k1=k1, v1=v1, n1=n1, kv1_batches=1,
+              bank_batches=bank_batches if n1 else 0)
+    return q, kv
+
+
+def case_attention_peaky(batch, heads, d, nq, n0, n1, pattern, bank_batches=None, seed=0):
     bb = batch if bank_batches is None else bank_batches
-    for b in range(batch):
-        qq = q[b * nq:(b + 1) * nq].float().reshape(nq, heads, d).transpose(0, 1)
-        kk = k0[b * n0:(b + 1) * n0].float()
-        vv = v0[b * n0:(b + 1) * n0].float()
-        if n1 and b < bb:
-            sl = slice(b * n1, (b + 1) * n1) if kv1_batches > 1 else slice(0, n1)
-            kk = torch.cat([kk, k1[sl].float()], 0)
-            vv = torch.cat([vv, v1[sl].float()], 0)
-        kk = kk.reshape(-1, heads, d).transpose(0, 1)
-        vv = vv.reshape(-1, heads, d).transpose(0, 1)
-        s = (qq @ kk.transpose(1, 2)) * d ** -0.5
-        o = s.softmax(-1) @ vv
-        refs.append(o.transpose(0, 1).reshape(nq, c))
-    ref = torch.cat(refs, 0)
-    return rel(out.float(), ref), 3e-3, (f"attention B={batch} h={heads} d={d} nq={nq} n0={n0} n1={n1} "
-                                          f"kv1b={kv1_batches} bank_b={bb}")
+    q, kv = attention_peaky_inputs(batch, heads, d, nq, n0, n1, pattern, bb, seed=seed)
+    ldv = (n0 + 7) // 8 * 8
+    kw = {}
+    if n1:
+        kw = dict(k1=kv["k1"], vt1=kv["v1"].t().contiguous(), n1=n1, kv1_batches=1, bank_batches=bb)
+    out = ops.attention(q, kv["k0"], _vt_padded(kv["v0"], batch, n0, ldv), n0, heads=heads, d=d, batch=batch, nq=nq,
+                        ldv0_batch=ldv, **kw)
+    ref = attention_ref(q, heads, d, batch, nq, **kv)
+    return rel(out.float(), ref), 3e-3, (f"attention {pattern} B={batch} h={heads} d={d} nq={nq} n0={n0} n1={n1} "
+                                          f"bank_b={bb}")
 
 
-def case_time_path(batch, seed=0):
+def case_time_path(batch, t_count=0, seed=0):
+    """t_count: 0 = one timestep per row, else t_count timesteps repeated over the rows (row b uses t[b % t_count])"""
     base = [981, 441, 1, 999, 500, 21, 7, 123]
-    t = torch.tensor([(base[i % 8] + 13 * (i // 8)) % 1000 for i in range(batch)], dtype=torch.long, device=DEV)
-    emb = ops.timestep_embedding(t, 320)
+    nt = t_count or batch
+    t = torch.tensor([(base[i % 8] + 13 * (i // 8)) % 1000 for i in range(nt)], dtype=torch.long, device=DEV)
+    emb = ops.timestep_embedding(t, 320, rows=batch)
     half = 160
     freqs = torch.exp(-math.log(10000) * torch.arange(half, dtype=torch.float32, device=DEV) / half)
-    args = t[:, None].float() * freqs[None]
+    args = t[torch.arange(batch, device=DEV) % nt, None].float() * freqs[None]
     ref = torch.cat([torch.cos(args), torch.sin(args)], -1)
     e1 = float((emb - ref).abs().max())
     w = _rand(1280, 320, seed=seed, scale=320 ** -0.5).half()
     b = _rand(1280, seed=seed + 1).float()
     out = ops.skinny_linear(ref, w, b, silu_in=True, silu_out=True)
     r2 = F.silu(F.silu(ref) @ w.float().t() + b)
-    return max(e1, rel(out, r2)), 1e-4, f"timestep embedding + skinny linear B={batch}"
+    return max(e1, rel(out, r2)), 1e-4, f"timestep embedding + skinny linear B={batch} timesteps={nt}"
 
 
-def case_layout(batch, c, h, w, seed=0):
+def case_layout(batch, c, h, w, copies=1, seed=0):
+    """copies > 1: the NHWC result repeats the batch (the cond | uncond pair); bit-exact"""
     x = _rand(batch, c, h, w, seed=seed)
-    y = ops.nchw_f32_to_nhwc_f16(x)
-    ref = x.half().permute(0, 2, 3, 1).reshape(-1, c)
-    e1 = float((y.float() - ref.float()).abs().max())
-    z = ops.nhwc_f16_to_nchw_f32(y, batch=batch, c=c, h=h, w=w)
+    y = ops.nchw_f32_to_nhwc_f16(x, copies=copies)
+    ref = x.half().permute(0, 2, 3, 1).reshape(-1, c).repeat(copies, 1)
+    e1 = float((y.float() - ref.float()).abs().max()) if y.shape == ref.shape else float("inf")
+    z = ops.nhwc_f16_to_nchw_f32(y[:batch * h * w], batch=batch, c=c, h=h, w=w)
     e2 = float((z - x.half().float()).abs().max())
-    return e1 + e2, 0.0, f"layout converts B={batch} c={c} {h}x{w}"
+    return e1 + e2, 0.0, f"layout converts B={batch} c={c} {h}x{w} copies={copies}"
 
 
 def case_add(batch, n, bcast, seed=0):
@@ -289,16 +431,50 @@ def case_add(batch, n, bcast, seed=0):
     return float((out.float() - ref.float()).abs().max()), 0.0, f"add B={batch} n={n} bcast={bcast}"
 
 
-def case_cfg_ddim(seed=0):
-    x, ec, eu = (_rand(2, 4, 64, 64, seed=seed + i) for i in range(3))
-    a_t, a_prev, sigma, scale = 0.0047, 0.0058, 0.0, 7.0
+def case_cfg_ddim(sigma=0.0, update_x=False, seed=0):
+    """sigma > 0: the stochastic DDIM step (noise added); update_x: x is overwritten with x_prev in place, and
+    pred_x0 must still come from the old x"""
+    x, ec, eu, noise = (_rand(2, 4, 64, 64, seed=seed + i) for i in range(4))
+    x_old = x.clone()
+    a_t, a_prev, scale = 0.0047, 0.0058, 7.0
     coef = torch.tensor([scale, math.sqrt(a_t), math.sqrt(a_prev), math.sqrt(1 - a_prev - sigma ** 2), sigma,
                          math.sqrt(1 - a_t)], dtype=torch.float32, device=DEV)
-    xp, p0 = ops.cfg_ddim_update(x, ec, eu, coef)
+    xp, p0 = ops.cfg_ddim_update(x, ec, eu, coef, noise=noise if sigma > 0 else None, update_x=update_x)
+    xo, ec, eu, noise = (t.double() for t in (x_old, ec, eu, noise))
     e = eu + scale * (ec - eu)
-    rp0 = (x - math.sqrt(1 - a_t) * e) / math.sqrt(a_t)
-    rxp = math.sqrt(a_prev) * rp0 + math.sqrt(1 - a_prev) * e
-    return max(rel(xp, rxp), rel(p0, rp0)), 1e-5, "cfg + ddim update"
+    rp0 = (xo - math.sqrt(1 - a_t) * e) / math.sqrt(a_t)
+    rxp = math.sqrt(a_prev) * rp0 + math.sqrt(1 - a_prev - sigma ** 2) * e + sigma * noise * (sigma > 0)
+    err = max(rel(xp, rxp), rel(p0, rp0))
+    if not torch.equal(x, xp if update_x else x_old):
+        err = float("inf")  # x must hold x_prev exactly (update_x) or be left alone
+    return err, 1e-5, f"cfg + ddim update sigma={sigma} update_x={update_x}"
+
+
+def case_softmax_rows(rows, cols, ld, scale=1.0, seed=0):
+    """in-place row softmax (VAE attention) against float64; row 0 peaky, row 1 constant; the pitch gap
+    [cols, ld) must stay untouched"""
+    x = (_rand(rows, ld, seed=seed) * 3).half()
+    x[0, :cols] = -4.0
+    x[0, cols // 3] = 30.0
+    x[1, :cols] = 2.5
+    before = x.clone()
+    ref = (x[:, :cols].double() * scale).softmax(-1)
+    ops.softmax_rows(x[:, :cols], scale=scale)
+    err = rel(x[:, :cols].float(), ref)
+    if not torch.equal(x[:, cols:], before[:, cols:]):
+        err = float("inf")
+    return err, 1e-3, f"softmax rows={rows} cols={cols} ld={ld} scale={scale}"
+
+
+def case_im2col_br(batch, h, w, c, seed=0):
+    """im2col for the VAE encoder's Downsample: pad (0, 1, 0, 1), 3x3 window, stride 2; bit-exact"""
+    x = _rand(batch, c, h, w, seed=seed).half()
+    xn = x.permute(0, 2, 3, 1).contiguous().reshape(batch * h * w, c)
+    col = ops.im2col3x3(xn, batch=batch, h=h, w=w, c=c, stride=2, pad="br")
+    u = F.unfold(F.pad(x.float(), (0, 1, 0, 1)), 3, stride=2)  # [B, c*9, L], column order (channel, ky, kx)
+    ref = u.reshape(batch, c, 9, -1).permute(0, 3, 2, 1).reshape(-1, 9 * c)
+    err = float((col.float() - ref).abs().max()) if col.shape == ref.shape else float("inf")
+    return err, 0.0, f"im2col 3x3 stride 2 pad (0,1,0,1) B={batch} {h}x{w} c={c}"
 
 
 ALL_CASES = [
@@ -438,4 +614,43 @@ ALL_CASES = [
     (case_tuned, (ATT2Q, case_attention, 2, 8, 80, 1024, 77, 0, 1, None, True)),
     (case_tuned, (ATT2Q, case_attention, 1, 8, 80, 384, 384, 128, 1)),        # odd number of Q tiles
     (case_attention, (16, 8, 80, 1024, 1024, 1024, 1, 8)),   # 1024 CTAs: picked by the heuristics
+    # ---- hot-path layouts: fused Q|K projection, one text context for the batch, output slice of a wider buffer ----
+    (case_attention, (2, 8, 40, 1024, 1024, 0, 1, None, False, "qk_fused")),
+    (case_attention, (2, 8, 80, 256, 256, 0, 1, None, False, "qk_fused+wide_out")),
+    (case_attention, (2, 8, 160, 64, 64, 0, 1, None, False, "qk_fused")),
+    (case_tuned, (ATT2Q, case_attention, 2, 8, 40, 1024, 1024, 0, 1, None, False, "qk_fused+wide_out")),
+    (case_tuned, (ATT2Q, case_attention, 2, 8, 80, 384, 384, 0, 1, None, False, "qk_fused")),
+    (case_attention, (2, 8, 40, 1024, 77, 0, 1, None, True, "shared_kv")),
+    (case_attention, (2, 8, 80, 256, 77, 0, 1, None, True, "shared_kv+wide_out")),
+    (case_attention, (2, 8, 160, 256, 77, 0, 1, None, True, "shared_kv")),
+    (case_tuned, (ATT2Q, case_attention, 2, 8, 40, 1024, 77, 0, 1, None, True, "shared_kv")),
+    (case_tuned, (ATT2Q, case_attention, 2, 8, 80, 256, 77, 0, 1, None, True, "shared_kv")),
+    (case_attention, (2, 8, 160, 256, 200, 64, 1, 1, False, "wide_out")),
+    (case_layout, (2, 4, 64, 64, 2)),
+    (case_layout, (1, 4, 24, 40, 2)),
+    (case_time_path, (16, 8)),                 # cond | uncond: rows 8..15 repeat the eight timesteps
+    (case_time_path, (6, 1)),                  # one timestep for the whole batch
+    (case_cfg_ddim, (0.05,)),                  # stochastic step: sigma * noise
+    (case_cfg_ddim, (0.0, True)),              # x advances in place
+    (case_cfg_ddim, (0.05, True)),
+    (case_softmax_rows, (64, 8, 8)),
+    (case_softmax_rows, (16, 4096, 4096)),
+    (case_softmax_rows, (32, 1000, 1000)),     # not a multiple of 256 threads x 8
+    (case_softmax_rows, (8, 2056, 2112)),      # row pitch > cols
+    (case_softmax_rows, (16, 4096, 4160, 0.125)),
+    (case_im2col_br, (2, 9, 7, 64)),
+    (case_im2col_br, (1, 8, 8, 128)),
+    (case_im2col_br, (1, 32, 30, 128)),
 ]
+
+# ---- online-softmax rescale path: every peaky pattern on every attention kernel ----
+# (pattern, n0, n1, bank_batches); all with B=2, 2 heads, 256 queries (two Q tiles)
+PEAKY_SHAPES = [("rise", 640, 0, None), ("slow_rise", 768, 0, None), ("mixed_rows", 512, 0, None),
+                ("fall", 640, 0, None), ("bank_peak", 256, 128, 1), ("ragged_peak", 77, 0, None),
+                ("ragged_peak", 200, 0, None)]
+PEAKY_KERNELS = [(None, 160), (None, 40), (None, 80), (ATT2Q, 40), (ATT2Q, 80)]  # attn_tc, attn3 x2, attn2 x2
+for _tune, _d in PEAKY_KERNELS:
+    for _pat, _n0, _n1, _bb in PEAKY_SHAPES:
+        _args = (2, 2, _d, 256, _n0, _n1, _pat, _bb)
+        ALL_CASES.append((case_attention_peaky, _args) if _tune is None else
+                         (case_tuned, (_tune, case_attention_peaky) + _args))
